@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- decode tokens/sec of a LLaMA-7B-shaped model over the quantised KV cache (BASELINE.json's metric).
 
-    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one batch-1 decode step at cache length L of the named workload: for every layer q/k/v projection,
 fused device-side append (NUQ quantise + top-K outlier split + pack), fused attend over the packed cache
@@ -33,6 +33,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark writes nothing into the tree it runs from: without this, its first import of modules that build()
+# does not import (kvquant_b200.decode, .synth, .p2p) would add __pycache__/ files there
+sys.dont_write_bytecode = True
 
 WORKLOADS = {
     # name: (model, bits, L (quantised slots), n_sink, outliers, description = BASELINE.json configs[i])
@@ -324,7 +327,15 @@ def main():
                          "theirs and merges (validated against NCCL at 2/4/8 GPUs, tests/test_zz_p2p_exchange.py); "
                          "nccl: all_gather + merge kernel")
     ap.add_argument("--torch-profile", default="", help="write a per-kernel table of 3 graph replays to this file (diagnostic)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the logits the last timed step returned to the host as "
+                         "DIR/logits.npy (float32); weights, caches and tokens are seeded, so the same arguments "
+                         "give the same inputs and two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the decode step's logits: it needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     import numpy as np
@@ -512,6 +523,10 @@ def main():
         step_e2e(i)
     ms_e2e = timed(step_e2e, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the last timed step is step_e2e(steps - 1): its logits sit in pinned host memory, synchronised
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "logits.npy"), pinned_logits.float().numpy())
     if sp_mode and stage.xchg is not None:
         bad = torch.tensor([1 if stage.xchg.failed() else 0], device=dev)
         dist.all_reduce(bad, op=dist.ReduceOp.MAX)

@@ -8,7 +8,6 @@ import subprocess
 import sys
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -46,20 +45,29 @@ def test_host_generated_layer_has_the_cache_layout():
     assert 1 <= n <= len(os.sched_getaffinity(0)) and "affinity" in desc
 
 
-def test_reference_class_extraction_is_verbatim():
+def test_reference_class_extraction_is_verbatim(tmp_path):
     import build_ref_py
-    if not os.path.exists(build_ref_py.SRC):
-        pytest.skip("/root/reference not present")
-    assert build_ref_py.build()
-    out = open(build_ref_py.OUT).read()
+    # a module laid out like the reference's modeling_llama.py: the three wanted definitions among others,
+    # a decorator, comments, blank lines and odd spacing that a re-rendering of the AST would not keep
+    src_path, out_path = tmp_path / "modeling_llama.py", tmp_path / "_ref" / "ref_cache_managers.py"
+    src_path.write_text(
+        "import torch\n\nclass LlamaRMSNorm:\n    pass\n\n\n"
+        "@torch.no_grad()\ndef compute_lut(x,  y):   # two spaces kept\n    return (x +\n            y)\n\n"
+        "def unrelated():\n    return 1\n\n"
+        "class QuantK(object):\n    '''doc'''\n\n    def f(self):\n        return 0x10  # hex kept\n\n"
+        "X = 3\n\nclass QuantV:\n    a = [1,\n         2]\n")
+    assert build_ref_py.build(src=str(src_path), out=str(out_path))
+    out = out_path.read_text()
     tree = ast.parse(out)
     names = [n.name for n in tree.body if isinstance(n, (ast.FunctionDef, ast.ClassDef))]
     assert names == ["compute_lut", "QuantK", "QuantV"]
-    src = open(build_ref_py.SRC).read().splitlines(keepends=True)
+    src = src_path.read_text().splitlines(keepends=True)
     ref_tree = ast.parse("".join(src))
     for node in ref_tree.body:
         if isinstance(node, (ast.FunctionDef, ast.ClassDef)) and node.name in build_ref_py.WANTED:
-            assert "".join(src[node.lineno - 1:node.end_lineno]) in out      # byte for byte
+            first = min([node.lineno] + [d.lineno for d in node.decorator_list])
+            assert "".join(src[first - 1:node.end_lineno]) in out      # byte for byte
+    assert "unrelated" not in out and "LlamaRMSNorm" not in out
     # the generated file lives in the git-ignored oracle/_ref/ only
     assert os.path.dirname(build_ref_py.OUT).endswith(os.path.join("oracle", "_ref"))
     rc = subprocess.run(["git", "check-ignore", "-q", build_ref_py.OUT], cwd=ROOT).returncode
